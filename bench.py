@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run)
     python bench.py --impl reference ...                     (the path's CPU implementation, timed alone)
+    python bench.py ... --dump-outputs DIR                   (also writes the last timed step's outputs: dump_outputs())
 
 A *step* is one pass of the hot path over one batch of synthetic input: every rank renders its
 `--views-per-rank` camera views of the SAME replicated gaussians forward + backward (L1 loss against a
@@ -47,6 +48,7 @@ for _p in (ROOT, PKG):
 METRIC = "fwd+bwd Mpix/s @1M gaussians 1080p"
 UNIT = "Mpix/s"
 LOG_SCALE_MEAN = -5.3   # mean reference tiles-touched per visible gaussian ~= 7 (SURVEY.md 8d asks 4-8)
+DUMP_ROWS = 65536       # gaussians sampled by --dump-outputs: 119 floats each at most (59 gradients, 59 parameters, radius) = 31 MB
 
 
 def parse():
@@ -88,7 +90,39 @@ def parse():
     ap.add_argument("--iterations", type=int, default=1000, help="train6m: iterations")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-baseline-seconds", type=float, default=20.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the device-resident timed steps, write what the last of them returned to its caller as DIR/<name>.npy "
+                         "(see dump_outputs), so that two builds can be compared on identical inputs")
+    a = ap.parse_args()
+    if a.dump_outputs and (a.impl != "ours" or a.workload != "raster"):
+        ap.error("--dump-outputs applies to the rasterizer workload of this implementation (--impl ours --workload raster)")
+    return a
+
+
+def dump_outputs(directory, last, pc, with_params):
+    """Writes what the caller of the last timed step received: the per-view losses (losses.npy, [V]) and, per gaussian, the
+    largest screen radius over the step's views (radii_max.npy) and the gradient of each rasterizer input (grad_means3D.npy,
+    grad_shs.npy, grad_opacities.npy, grad_scales.npy, grad_rotations.npy); with --optimizer also the inputs as the optimizer
+    step left them (means3D.npy, ...).  Per-gaussian arrays hold a sample of DUMP_ROWS gaussians drawn with a fixed seed, so
+    the same --gaussians gives the same rows; gaussian_index.npy lists them (float64), every other array is float32."""
+    import numpy as np
+    import torch
+    inputs = {"means3D": pc.get_xyz, "shs": pc.get_features, "opacities": pc.get_opacity, "scales": pc.get_scaling,
+              "rotations": pc.get_rotation}
+    P = int(pc.get_xyz.shape[0])
+    rows = torch.arange(P) if P <= DUMP_ROWS else \
+        torch.randperm(P, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    idx = rows.to(pc.get_xyz.device)
+    arrays = {"gaussian_index": rows.double(), "losses": torch.stack(list(last["losses"])),
+              "radii_max": torch.stack(last["radii"]).amax(dim=0)[idx]}
+    for name, t in inputs.items():
+        arrays["grad_" + name] = t.grad[idx]
+        if with_params:
+            arrays[name] = t.detach()[idx]
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        np.save(os.path.join(directory, name + ".npy"), t.numpy() if t.dtype == torch.float64 else t.float().numpy())
 
 
 class BenchCamera:
@@ -501,6 +535,7 @@ def main():
 
     loss_host = torch.zeros(1024, 1).pin_memory()
     step_counter = [0]
+    last = {}                       # per-view losses and radii the latest step returned (--dump-outputs)
 
     def step(host_inputs: bool):
         if a.api != "views":
@@ -529,6 +564,7 @@ def main():
                                         capacity=capacity, grad_chunks=grad_chunks if chunked else 1,
                                         on_grad_chunk=on_chunk if chunked else None,
                                         peers=peer_bucket.table() if peer_bucket is not None else None)
+            last["losses"], last["radii"] = out["losses"], [out["radii_max"]]
             total = out["losses"].sum()
             if peer_bucket is not None:
                 peer_bucket.finish()        # barrier + in-place all-gather of the owned rows: every rank holds the summed gradient
@@ -539,6 +575,7 @@ def main():
                 bucket.all_reduce()
         else:
             total = torch.zeros((), device=dev)
+            last["losses"], last["radii"] = [], []
             for i, cam in enumerate(cams):
                 if host_inputs:
                     cam.upload(dev)
@@ -549,6 +586,8 @@ def main():
                 loss = (pkg["render"] - gt).abs().mean()
                 loss.backward()
                 total += loss.detach()
+                last["losses"].append(loss.detach())
+                last["radii"].append(pkg["radii"])
             bucket.all_reduce()
         if a.optimizer:
             pc.update_learning_rate(pc.step_count + 1)
@@ -648,6 +687,8 @@ def main():
     dgr.set_option("time_kernels", 0)
     clocks = sampler.stop() if rank == 0 else None
     value = mpix_step * a.steps / (ms_total / 1e3)
+    if a.dump_outputs and rank == 0:      # before the next leg's steps overwrite the gradients
+        dump_outputs(a.dump_outputs, last, pc, with_params=a.optimizer)
 
     # ---- end-to-end leg (host inputs) ----
     for _ in range(max(a.warmup, 3)):
@@ -670,7 +711,7 @@ def main():
         for i in range(2 * V):
             one_view(i)
         torch.cuda.synchronize()
-        n_sv = max(V, min(a.steps * V, 64))
+        n_sv = a.steps * V
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         gc.collect(); gc.disable()
         e0.record()

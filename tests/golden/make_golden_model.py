@@ -49,7 +49,7 @@ opt = OptimizationParams(ArgumentParser())
 out = {}
 
 g = torch.Generator().manual_seed(4321)
-P0, EXTENT = 300, 4.0
+P0, EXTENT = 64, 4.0          # ten full snapshots of parameters and both Adam moments: the fixture stays under 1 MB
 pc = GM.GaussianModel(3)
 pc.active_sh_degree = 3
 pc.spatial_lr_scale = EXTENT
